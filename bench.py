@@ -2,8 +2,9 @@
 """bench.py -- throughput of the two WaveNet hot paths on B200, with roofline and the CPU baseline beside it.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload all|generate|train]
+                    [--dump-outputs DIR]
 
-Under torchrun (N>1) every rank runs; rank 0 prints ONE JSON line.
+Under torchrun (N>1) every rank runs; rank 0 prints ONE JSON line.  Every timed loop runs --steps iterations.
 
 Primary metric (BASELINE.json configs[1]): generate_fast samples/sec -- layers=10, blocks=5, 256 channels,
 16000 samples (1 s of 16 kHz audio), single stream; a "step" is one full generate_fast run.  At N>1 each rank runs
@@ -13,6 +14,11 @@ L=16000, output_length=10885), batch-sharded over the ranks (weak scaling; the f
 
 `value` is device-timed with inputs resident in HBM; `e2e` goes through the reference-facing Python API with host
 buffers.  `cpu_baseline` / `--impl reference` time the CPU port of the reference (oracle/) on the host cores.
+
+`--dump-outputs DIR` (e.g. bench_outputs/, which git ignores) writes what the last timed step returned, as float32
+.npy files, so that two builds can be compared output for output (the inputs are seeded): DIR/generate_indices.npy,
+the (1, 16000) sampled class indices, and with the training forward DIR/train_logits.npy, a fixed seeded sample of
+TRAIN_DUMP_ROWS of its (87080, 256) logits, whose row numbers are in DIR/train_logits_rows.npy.
 """
 import argparse
 import json
@@ -37,6 +43,7 @@ GEN_KW = dict(layers=10, blocks=5, dilation_channels=256, residual_channels=256,
 GEN_SAMPLES = 16000
 TRAIN_B, TRAIN_L = 8, 16000
 TEMPERATURE = 1.0
+TRAIN_DUMP_ROWS = 8192
 GEN_WORKLOAD = ("cfg2 generate_fast: layers=10 blocks=5 ch=256 classes=256, 16000 samples, single stream, temperature=1.0, "
                 "seeded random-init weights")
 
@@ -154,8 +161,14 @@ class L2Flush:
         self.buf.fill_(1)
 
 
+def write_outputs(path, arrays):
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------ generation
-def bench_generate(args, world, rank):
+def bench_generate(args, world, rank, dump=None):
     model = build_model(GEN_KW).cuda()
     rt = model._runtime()
     NS, n = 1, GEN_SAMPLES
@@ -186,6 +199,8 @@ def bench_generate(args, world, rank):
         evs.append((e0, e1))
     barrier_sync(world)
     t_wall = time.perf_counter() - t_wall0
+    if dump is not None:                  # before the argmax run below reuses `out`
+        dump["generate_indices"] = out.cpu().numpy().astype(np.float32)
     clk = clocks.stop()
     ms = sum(a.elapsed_time(b) for a, b in evs)
     ms = max_over_ranks(ms, world)
@@ -195,7 +210,7 @@ def bench_generate(args, world, rank):
     model.generate_fast(256, temperature=TEMPERATURE)                     # warm
     barrier_sync(world)
     t0 = time.perf_counter()
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     for _ in range(e2e_steps):
         audio = model.generate_fast(n, temperature=TEMPERATURE)
     torch.cuda.synchronize()
@@ -208,7 +223,7 @@ def bench_generate(args, world, rank):
     import ctypes, native
     # argmax path, for reference
     t_arg = []
-    for _ in range(2):
+    for _ in range(args.steps):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         rt.generate_resident(s, first, 1, n, 0.0, 0.0, out)
@@ -226,7 +241,7 @@ def bench_generate(args, world, rank):
         out_b = torch.zeros(NB, nb, dtype=torch.int32, device=dev)
         rt.generate_resident(sb, first_b, 1, 64, TEMPERATURE, 0.0, out_b[:, :64].contiguous(), d_uni=uni_b[:, :64].contiguous())
         tb = []
-        for _ in range(2):
+        for _ in range(args.steps):
             flush()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
@@ -246,7 +261,7 @@ def bench_generate(args, world, rank):
         out_b = torch.zeros(NB, nb, dtype=torch.int32, device=dev)
         rt.generate_resident(sb, first_b, 1, 64, TEMPERATURE, 0.0, out_b[:, :64].contiguous(), d_uni=uni_b[:, :64].contiguous())
         tb = []
-        for _ in range(2):
+        for _ in range(args.steps):
             flush()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
@@ -316,7 +331,7 @@ def train_alg_bytes(model, B, L, dense_input):
     return per_layer, start, head, flops
 
 
-def bench_train(args, world, rank):
+def bench_train(args, world, rank, dump=None):
     kw = dict(GEN_KW)
     model = build_model(kw).cuda()
     rt = model._runtime()
@@ -343,6 +358,10 @@ def bench_train(args, world, rank):
         rt.block_events = None
         barrier_sync(world)
         clk = clocks.stop()
+        if dump is not None:
+            rows = torch.randperm(y.shape[0], generator=torch.Generator().manual_seed(0))[:TRAIN_DUMP_ROWS].sort().values
+            dump["train_logits_rows"] = rows.numpy().astype(np.float32)
+            dump["train_logits"] = y[rows.to(y.device)].float().cpu().numpy()
         fwd_mode = getattr(rt, "last_block_mode", "ffma")
         ms = max_over_ranks(sum(a.elapsed_time(b) for a, b in evs), world)
         block_ms = sum(a.elapsed_time(b) for a, b in bevs) / args.steps
@@ -354,7 +373,7 @@ def bench_train(args, world, rank):
         model(x_host.cuda(non_blocking=True))
         barrier_sync(world)
         t0 = time.perf_counter()
-        e2e_steps = max(1, min(args.steps, 3))
+        e2e_steps = args.steps
         for _ in range(e2e_steps):
             y = model(x_host.cuda(non_blocking=True))
             y_host.copy_(y, non_blocking=True)
@@ -382,7 +401,7 @@ def bench_train(args, world, rank):
             for _ in range(2):
                 y_fast = model.forward_indices(d_idx)
             fe = []
-            for _ in range(max(1, min(args.steps, 3))):
+            for _ in range(args.steps):
                 flush()
                 b0, b1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 rt.block_events = (b0, b1)
@@ -408,7 +427,7 @@ def bench_train(args, world, rank):
             for _ in range(2):
                 y_other = model.forward_indices(d_idx)
             oe = []
-            for _ in range(max(1, min(args.steps, 3))):
+            for _ in range(args.steps):
                 flush()
                 b0, b1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 rt.block_events = (b0, b1)
@@ -427,7 +446,7 @@ def bench_train(args, world, rank):
     red = dp.make_data_parallel(model)
     target = torch.randint(0, 256, (B * model.output_length,), generator=torch.Generator().manual_seed(99 + rank)).cuda()
     step_ms = []
-    for i in range(1 + max(1, min(args.steps, 3))):
+    for i in range(1 + args.steps):
         model.zero_grad(set_to_none=True)
         barrier_sync(world)
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -453,7 +472,7 @@ def bench_train(args, world, rank):
         mine = dp.shard_batch(sidx, rank, world).to(torch.uint8).cuda()
         mine_t = dp.shard_batch(stgt, rank, world).reshape(-1).cuda()
         sms = []
-        for i in range(3):
+        for i in range(1 + args.steps):
             model.zero_grad(set_to_none=True)
             barrier_sync(world)
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -564,7 +583,7 @@ def bench_train_cfg5(args, world, rank):
     idx = torch.randint(0, 256, (1, L), generator=torch.Generator().manual_seed(4321 + rank)).to(torch.uint8).cuda()
     target = torch.randint(0, 256, (model.output_length,), generator=torch.Generator().manual_seed(55 + rank)).cuda()
     flush = L2Flush()
-    n = max(1, min(args.steps, 3))
+    n = args.steps
     with torch.no_grad():
         for _ in range(2):
             model.forward_indices(idx)
@@ -710,14 +729,18 @@ def main():
     ap.add_argument("--no-batched", action="store_true", help="skip the 64-stream (cfg4) generation figure")
     ap.add_argument("--no-cfg5", action="store_true", help="skip the 512-channel bf16 deep-stack figures (cfg 5)")
     ap.add_argument("--variants", action="store_true", help="also time the other operand splits of the two-launch blocks")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device (the B200 path has no CPU fallback); use --impl reference for the CPU arm")
     world, rank, _ = dist_setup(args.gpus)
-    gen = bench_generate(args, world, rank) if args.workload in ("all", "generate") else None
-    train = bench_train(args, world, rank) if args.workload in ("all", "train") else None
+    dump = {} if args.dump_outputs and rank == 0 else None
+    gen = bench_generate(args, world, rank, dump) if args.workload in ("all", "generate") else None
+    train = bench_train(args, world, rank, dump) if args.workload in ("all", "train") else None
     cfg5 = None
     if train is not None and not args.no_cfg5:
         torch.cuda.empty_cache()
@@ -789,6 +812,8 @@ def main():
                 summ.update(cfg5_fwd_ms=train["cfg5"]["ms_per_step"], cfg5_step_ms=train["cfg5"]["train_step"]["ms_per_step"],
                             cfg5_tensor_frac=train["cfg5"]["roofline"]["frac"])
         line["summary"] = summ
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         print(json.dumps(line))
     if world > 1:
         import torch.distributed as dist

@@ -1,9 +1,7 @@
 #!/usr/bin/env python
 """Generate the golden fixtures in this directory by running the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference, which does not exist on the GPU box):
-
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <checkout of the original pytorch-wavenet>
 
 The reference sources are imported from where they lie (nothing is copied); five compatibility shims make
 the 2017 / torch-0.3 code run on torch 2.x (SURVEY.md section 8c):
@@ -13,9 +11,12 @@ the 2017 / torch-0.3 code run on torch 2.x (SURVEY.md section 8c):
   4. ``torch.max(x, 0)`` inside module ``wavenet_model`` returns a (1,1)-shaped index (no 0-dim tensors in 0.3;
      wavenet_model.py:292 does ``[1][0]``),
   5. the snapshot is loaded with ``weights_only=False`` and moved with ``.cpu()`` (wavenet_model.py:343-346).
-Everything written is a plain ``.npz`` of arrays.  The whole-object snapshot pickle is read once here and
-re-saved as a tensor-only state dict.
+Everything written is a plain ``.npz`` of arrays, each under 1 MB.  The seeded nets' weights are rebuilt from the seed
+by the tests, so only the small nets ship them; ``deep`` ships a SHA-256 per tensor instead.  The trained snapshot
+(1.83 M parameters) is re-saved with every tensor but the two head biases quantized to an 8-entry float32 codebook
+(``quantize``), and the reference runs on those weights, so its outputs here are exact for the stored weights.
 """
+import hashlib
 import os
 import sys
 import types
@@ -24,13 +25,12 @@ import numpy as np
 import torch
 import torch.nn.functional as F
 
-REF = "/root/reference"
 HERE = os.path.dirname(os.path.abspath(__file__))
 
 
-def import_reference():
+def import_reference(ref):
     sys.modules.setdefault("librosa", types.ModuleType("librosa"))                    # shim 1
-    sys.path.insert(0, REF)
+    sys.path.insert(0, ref)
     import wavenet_modules as wm                                                      # noqa: E402
     import wavenet_model as wmod                                                      # noqa: E402
 
@@ -65,6 +65,19 @@ def import_reference():
 
     wmod.torch = TorchProxy()
     return wm, wmod
+
+
+def quantize(w, levels=8, iters=25):
+    """(codebook, codes): 1-D k-means of the tensor's values, started at evenly spaced quantiles; codebook[codes] is
+    the float32 tensor the fixture stands for."""
+    x = w.detach().cpu().numpy().astype(np.float64).ravel()
+    book = np.quantile(x, (np.arange(levels) + 0.5) / levels)
+    for _ in range(iters):
+        codes = np.abs(x[:, None] - book[None, :]).argmin(1)
+        book = np.array([x[codes == j].mean() if np.any(codes == j) else book[j] for j in range(levels)])
+    book = book.astype(np.float32)
+    codes = np.abs(x[:, None] - book.astype(np.float64)[None, :]).argmin(1).astype(np.uint8)
+    return book, codes.reshape(tuple(w.shape))
 
 
 def state_arrays(model):
@@ -110,7 +123,10 @@ def audio_to_indices(audio, classes=256):
 
 
 def main():
-    wm, wmod = import_reference()
+    if len(sys.argv) != 2:
+        raise SystemExit(__doc__)
+    ref = sys.argv[1]
+    wm, wmod = import_reference(ref)
     torch.set_num_threads(8)
     out = {}
 
@@ -168,7 +184,9 @@ def main():
                     gen_sample_uniforms=u,
                     w_checksum=np.float64(sum(float(np.abs(v).astype(np.float64).sum()) for v in w.values())))
         arrs.update({"kw_" + k: v for k, v in kw.items()})
-        if name != "cfg1":
+        if name == "deep":                                    # rebuilt from the seed by the tests, checked per tensor
+            arrs.update({"d:" + k: np.array(hashlib.sha256(v.astype("<f4").tobytes()).hexdigest()) for k, v in w.items()})
+        elif name != "cfg1":
             arrs.update({"w:" + k: v for k, v in w.items()})  # small nets: ship the weights too
         np.savez_compressed(os.path.join(HERE, f"net_{name}.npz"), **arrs)
         out[name] = (fwd.shape, float(fwd.abs().max()))
@@ -197,14 +215,22 @@ def main():
     out["cfg2"] = (fwd.shape, float(np.abs(fwd.numpy()).max()))
 
     # ---------------- the shipped trained snapshot on real mu-law audio
-    snap = os.path.join(REF, "snapshots", "chaconne_model_2017-12-28_16-44-12")
+    snap = os.path.join(ref, "snapshots", "chaconne_model_2017-12-28_16-44-12")
     m = torch.load(snap, map_location="cpu", weights_only=False)                      # shim 5
     m.cpu()
-    sd = state_arrays(m)
-    np.savez(os.path.join(HERE, "snapshot_chaconne_state.npz"), layers=m.layers, blocks=m.blocks,
-             kernel_size=m.kernel_size, classes=m.classes, output_length=m.output_length,
-             receptive_field=m.receptive_field, **{"w:" + k: v for k, v in sd.items()})
-    data = np.load(os.path.join(REF, "train_samples", "bach_chaconne", "dataset.npz"))["arr_0"]
+    packed = {}
+    with torch.no_grad():
+        for k, v in m.state_dict().items():
+            if k in ("end_conv_1.bias", "end_conv_2.bias"):      # exact, so that no two classes' logits tie exactly
+                packed["w:" + k] = v.numpy().copy()
+                continue
+            book, codes = quantize(v)
+            v.copy_(torch.from_numpy(book[codes.astype(np.int64)]))
+            packed["l:" + k], packed["c:" + k] = book, codes
+    np.savez_compressed(os.path.join(HERE, "snapshot_chaconne_state.npz"), layers=m.layers, blocks=m.blocks,
+                        kernel_size=m.kernel_size, classes=m.classes, output_length=m.output_length,
+                        receptive_field=m.receptive_field, **packed)
+    data = np.load(os.path.join(ref, "train_samples", "bach_chaconne", "dataset.npz"))["arr_0"]
     rf = m.receptive_field
     off = 960000
     clip = data[off:off + rf + 260].astype(np.int64)          # rf given samples + 260 for teacher forcing

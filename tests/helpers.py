@@ -1,4 +1,6 @@
 """Helpers shared by the parity tests (oracle side only; nothing here is product code)."""
+import hashlib
+
 import numpy as np
 import torch
 
@@ -14,7 +16,18 @@ def spec_from_golden(g, output_length=None):
 
 
 def params_from_golden(g):
-    return {k[2:]: torch.from_numpy(g[k]) for k in g.files if k.startswith("w:")}
+    """The weights a fixture stands for ({} if none): stored ("w:"), stored as a float32 codebook and codes ("l:", "c:";
+    the quantized snapshot), or rebuilt from seed 0 and checked against the reference's per-tensor SHA-256 ("d:")."""
+    digests = {k[2:]: str(g[k]) for k in g.files if k.startswith("d:")}
+    if digests:
+        p = O.init_params(spec_from_golden(g), seed=0)
+        assert set(p) == set(digests)
+        for k, v in p.items():
+            assert hashlib.sha256(v.numpy().astype("<f4").tobytes()).hexdigest() == digests[k], k
+        return p
+    p = {k[2:]: torch.from_numpy(g[k]) for k in g.files if k.startswith("w:")}
+    p.update({k[2:]: torch.from_numpy(g["l:" + k[2:]][g[k].astype(np.int64)]) for k in g.files if k.startswith("c:")})
+    return p
 
 
 def weight_checksum(params):

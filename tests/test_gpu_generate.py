@@ -56,7 +56,7 @@ def test_generate_snapshot_real_audio(golden):
     clip = gio["clip"].astype(np.int64)
     idx = m.generate_fast_batch(200, clip[None, :rf], temperature=0.0)
     n_ok = assert_stream_parity(idx[0], gio["gen_argmax_idx"], gio["gen_argmax_logits"])
-    assert n_ok >= 8 and idx[0][:8].tolist() == [178, 174, 169, 160, 148, 155, 174, 183]
+    assert n_ok >= 8 and idx[0][:8].tolist() == [177, 177, 177, 174, 174, 177, 181, 188]
     _, logits = m.generate_fast_batch(200, clip[None, :rf], temperature=0.0, forced=gio["gen_argmax_idx"][None, :],
                                       return_logits=True)
     assert rel_err(logits[0], gio["gen_argmax_logits"]) < TOL

@@ -1,7 +1,9 @@
 """Host-side logic that needs no GPU: constructor / state_dict compatibility, shape planning, the C ABI surface."""
 import ctypes
+import hashlib
 import os
 import re
+import struct
 
 import numpy as np
 import pytest
@@ -101,21 +103,35 @@ def test_snapshot_state_loads(golden):
     assert m.parameter_count() == 1834592 and m.receptive_field == 3070
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/snapshots/chaconne_model_2017-12-28_16-44-12"),
-                    reason="reference checkout not present (build container only)")
-def test_reference_pickle_unpickles_into_this_class():
+def test_reference_pickle_unpickles_into_this_class(golden, tmp_path):
     """The reference snapshots are whole-object pickles of wavenet_model.WaveNetModel; with this package on the
-    path they restore into THIS class (wavenet_model.py:330-346 load_latest_model_from / load_to_cpu)."""
-    m = wmod.load_to_cpu("/root/reference/snapshots/chaconne_model_2017-12-28_16-44-12")
+    path they restore into THIS class (wavenet_model.py:330-346 load_latest_model_from / load_to_cpu).  The chaconne
+    snapshot is reassembled from its stored pickle header, each storage filled from the stored parameters or with zeros
+    (tests/golden/make_golden_pickle.py)."""
+    gp = golden("snapshot_chaconne_pickle.npz")
+    p = params_from_golden(golden("snapshot_chaconne_state.npz"))
+    head = gp["head"].tobytes()
+    assert hashlib.sha256(head).hexdigest() == str(gp["head_sha256"])
+    path = tmp_path / "chaconne_model"
+    with open(path, "wb") as f:
+        f.write(head)
+        for src, n in zip(gp["sources"], gp["counts"]):
+            f.write(struct.pack("<q", int(n)))
+            f.write(p[str(src)].numpy().astype("<f4").tobytes() if src else bytes(4 * int(n)))
+    m = wmod.load_to_cpu(str(path))
     assert type(m) is wmod.WaveNetModel and m.receptive_field == 3070 and m.dtype == torch.FloatTensor
     assert type(m.dilated_queues[0]).__module__ == "wavenet_modules"
     assert m._runtime() is m._runtime()
+    assert set(m.state_dict()) == set(p) and all(torch.equal(v, p[k]) for k, v in m.state_dict().items())
 
 
-def test_no_cpu_fallback():
+def test_no_cpu_fallback(monkeypatch):
     m = wmod.WaveNetModel(layers=2, blocks=1, dilation_channels=4, residual_channels=4, skip_channels=4, end_channels=4)
     with torch.no_grad(), pytest.raises(RuntimeError, match="CUDA"):
         m(torch.zeros(1, 256, 16))
+    # generate_fast of a CPU-resident model samples on a CUDA copy when there is a device (test_gpu_generate covers
+    # that); without one it must raise rather than sample on the CPU
+    monkeypatch.setattr(torch.cuda, "is_available", lambda: False)
     with pytest.raises(RuntimeError, match="CUDA"):
         m.generate_fast(4)
     with pytest.raises(RuntimeError, match="CUDA"):
